@@ -5,6 +5,7 @@
     python bench.py --impl reference ...                                # the reference's own torch-CPU path (oracle port), all host cores
     python bench.py --impl torch-gpu ...                                # the reference's own GPU path: torch eager + cuDNN on this B200
                                                                         # (arms: fp32 NCDHW as shipped, bf16 autocast + channels_last_3d)
+    python bench.py --dump-outputs DIR ...                              # also write what the last timed step returned, DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for the definition of every field.  A "step" of the training
 workloads = zero grads, model(x, return_logits=True), BCEDiceLoss(logits, target), backward, gradient allreduce (N > 1); the optimizer
@@ -40,6 +41,8 @@ WORKLOADS = {
                  metric="UNet3D sliding-window inference patches/sec (128^3 patches, stride 64)"),
 }
 
+DUMP_MAX_ELEMS = 1 << 22   # 16 MB of float32 per dumped array; the training path writes three of them and the loss
+
 
 def parse():
     ap = argparse.ArgumentParser()
@@ -57,7 +60,29 @@ def parse():
     ap.add_argument("--buckets", type=int, default=4, help="gradient allreduce buckets (launched as backward finishes them)")
     ap.add_argument("--fused-loss", type=int, default=int(os.environ.get("B200UNET_FUSED_LOSS", "1")),
                     help="1: BCEDiceLoss through the engine's two-pass kernels (csrc/loss_ops.cu) instead of eager torch ops")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy in float32; "
+                         "an array of more than %d elements is written as a fixed seeded sample of its flattened values" % DUMP_MAX_ELEMS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 engine's path (--impl b200)")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy (float32).  Larger ones: the values at 2^22 flat indices drawn with a fixed seed
+    (sorted, duplicates dropped), so that two builds given the same arguments write comparable files."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).unique()
+            t = t.flatten()[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def peaks():
@@ -148,7 +173,7 @@ def run_reference(args, wl):
     inference = args.workload == "cfg5"
     # bounded sample: ONE patch of the workload's size per step (cfg4: 96^3 instead of 160^3 -- a 160^3 f64 step is ~minutes on CPU)
     sample_size = min(size, 96) if args.workload == "cfg4" else size
-    steps = min(args.steps, 3)
+    steps = args.steps
     warm = min(args.warmup, 1)
     sec, threads = cpu_reference_steps(wl, sample_size, 1, steps, warm, forward_only=inference)
     scale = (size / sample_size) ** 3  # FLOP-proportional extrapolation when the sample patch is smaller than the workload's
@@ -276,7 +301,14 @@ def run_train(args, wl):
         loss = P.losses.bce_dice_loss(logits, t, fused=bool(args.fused_loss))
         loss.backward()     # gradients land in flat.grad; each bucket's allreduce starts as soon as backward has written it
         reducer.finish()    # one sum-allreduce of every gradient per step over NVLink (replaces DataParallel's reduce-to-GPU-0)
-        return loss
+        return out, logits, loss
+
+    last = {}
+
+    def timed_step():
+        res = step(x_dev, t_dev)
+        if args.dump_outputs:
+            last["step"] = res
 
     def barrier():
         if world > 1:
@@ -308,9 +340,14 @@ def run_train(args, wl):
 
     # ---- timed region 1 (`value`): inputs resident in HBM, no instrumentation ----
     with ClockSampler(local) as clk:
-        ms = timed(lambda: step(x_dev, t_dev), args.steps)
+        ms = timed(timed_step, args.steps)
     patches = world * B * args.steps
     value = patches / (ms / 1e3)
+    if args.dump_outputs and rank == 0:   # before later steps overwrite the gradients (the engine writes them in place)
+        out, logits, loss = last.pop("step")
+        dump_outputs(args.dump_outputs, {"probabilities": out, "logits": logits, "loss": loss,
+                                         "param_grads": torch.cat([p.grad.flatten() for p in model.parameters()])})
+        del out, logits, loss
 
     # ---- timed region 2 (`e2e`): through the public nn.Module API with HOST buffers: pinned H2D of input + target on a copy stream,
     # double-buffered against the previous step's compute, loss read back every step (trainer.py:241) ----
@@ -330,7 +367,7 @@ def run_train(args, wl):
         torch.cuda.current_stream().wait_event(ev)
         xs.record_stream(torch.cuda.current_stream())
         ts.record_stream(torch.cuda.current_stream())
-        loss = step(xs, ts)
+        _, _, loss = step(xs, ts)
         stage()                 # the next step's H2D copies run while this step's kernels drain
         return loss.item()      # device -> host read of the loss
 
@@ -486,13 +523,22 @@ def run_predict(args, wl):
     def host_volume():     # host array in -> host array out: staging ring + H2D, patches, write-back, D2H
         return vp.predict(vol)
 
-    steps = max(1, min(args.steps, 5))
+    last = {}
+
+    def timed_volume():
+        out = device_volume()
+        if args.dump_outputs:
+            last["out"] = out
+
+    steps = args.steps
     W = max(args.warmup, 3)
     for _ in range(W):
         device_volume()
     with ClockSampler(local) as clk:
-        ms = timed(device_volume, steps)
+        ms = timed(timed_volume, steps)
     fwd_l, _ = P.last_launch_counts()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"probabilities": last.pop("out")})
     host_volume()
     t0 = time.perf_counter()
     ms_e2e = timed(host_volume, steps)

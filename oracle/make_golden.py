@@ -92,6 +92,16 @@ def run_block_case(name, module, x_shape, seed, extra_inputs=None):
     print(f"{name}: y {tuple(y.shape)}")
 
 
+def run_state_dict_case(name, cfg, seed, model_mod):
+    """The default-initialised state_dict of a model built by the reference's get_model under torch.manual_seed(seed): the
+    checkpoint a reference user would hand to the engine (names, order, shapes, values)."""
+    torch.manual_seed(seed)
+    m = model_mod.get_model(dict(cfg))
+    rec = {"sd/" + k: p.detach().numpy() for k, p in m.state_dict().items()}
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **rec)
+    print(f"{name}: {len(rec)} tensors")
+
+
 ONLY = None  # set by `--only name1,name2`: regenerate just these fixtures
 
 
@@ -100,12 +110,13 @@ def _wanted(name):
 
 
 def main():
-    global ONLY, run_model_case, run_block_case
+    global ONLY, run_model_case, run_block_case, run_state_dict_case
     if "--only" in sys.argv:
         ONLY = set(sys.argv[sys.argv.index("--only") + 1].split(","))
-        _rm, _rb = run_model_case, run_block_case
+        _rm, _rb, _rs = run_model_case, run_block_case, run_state_dict_case
         run_model_case = lambda name, *a, **k: _rm(name, *a, **k) if _wanted(name) else None  # noqa: E731
         run_block_case = lambda name, *a, **k: _rb(name, *a, **k) if _wanted(name) else None  # noqa: E731
+        run_state_dict_case = lambda name, *a, **k: _rs(name, *a, **k) if _wanted(name) else None  # noqa: E731
     os.makedirs(OUT, exist_ok=True)
     model_mod, bb, losses_mod = import_reference()
     torch.set_num_threads(1)  # reproducible reductions
@@ -181,6 +192,11 @@ def main():
     torch.manual_seed(19)
     run_block_case("block_decoder_deconv_32_16", bb.Decoder(32, 16, basic_module=bb.ResNetBlock), (1, 32, 4, 4, 4), 19,
                    extra_inputs=(1, 16, 8, 8, 8))
+
+    # ---- checkpoints (tests/test_boundary.py: a reference checkpoint loads into the engine and back) ----------------
+    run_state_dict_case("state_dict_resunetse3d_f16_l2_c2_seed3",
+                        dict(name="ResidualUNetSE3D", in_channels=1, out_channels=2, f_maps=16, num_levels=2, final_sigmoid=False),
+                        3, model_mod)
 
 
 if __name__ == "__main__":

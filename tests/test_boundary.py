@@ -1,50 +1,45 @@
-"""CPU: the drop-in boundary (SURVEY.md section 8(b)) -- install() against the REAL reference package when it is present in this
-container (/root/reference; the GPU box does not have it), constructor-time validation, nn.DataParallel replicas, flat
-parameter storage and gradient buckets."""
+"""CPU: the drop-in boundary (SURVEY.md section 8(b)) -- install() rebinding the reference package's model factory, checkpoint
+compatibility with the reference's state_dict (golden vectors from oracle/make_golden.py), constructor-time validation,
+nn.DataParallel replicas, flat parameter storage and gradient buckets."""
 import os
 import sys
 import types
 
+import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REF_MODEL = "pytorch3dunet.unet3d.model"
 
 
-def _stub(name, **attrs):
-    if name in sys.modules:
-        return
-    m = types.ModuleType(name)
-    for k, v in attrs.items():
-        setattr(m, k, v)
-    sys.modules[name] = m
+class _RefModel(torch.nn.Module):
+    """stand-in for a reference model class: records the keyword arguments it was constructed with"""
+
+    def __init__(self, **kwargs):
+        super().__init__()
+        self.kwargs = kwargs
 
 
 @pytest.fixture
 def reference_pkg():
-    """the reference package, importable with stand-ins for the optional dependencies this image lacks (skimage, h5py, imageio)"""
-    if not os.path.isdir(os.path.join(REF, "pytorch3dunet")):
-        pytest.skip("reference checkout not present (it never travels to the GPU box)")
-    _stub("skimage")
-    _stub("skimage.color", label2rgb=lambda *a, **k: None)
-    _stub("skimage.filters", gaussian=None)
-    _stub("skimage.segmentation", find_boundaries=None)
-    _stub("skimage.measure")
-    _stub("skimage.metrics", adapted_rand_error=None, peak_signal_noise_ratio=None, mean_squared_error=None)
-    _stub("h5py", Dataset=type("Dataset", (), {}), File=type("File", (), {}))
-    _stub("imageio")
-    added = REF not in sys.path
-    if added:
-        sys.path.insert(0, REF)
-    try:
-        import pytorch3dunet.unet3d.model as ref_model
-    except Exception as e:  # pragma: no cover
-        pytest.skip(f"reference not importable here: {e}")
+    """A stand-in for the reference's `pytorch3dunet.unet3d.model` with the surface install() works on: the model classes,
+    get_model (resolves the class by name in this module at call time and passes it the whole config, model.py:361-363) and
+    is_model_2d (model.py:366-369)."""
+    ref_model = types.ModuleType(REF_MODEL)
+    for name in ("UNet3D", "ResidualUNet3D", "ResidualUNetSE3D", "UNet2D", "ResidualUNet2D"):
+        setattr(ref_model, name, type(name, (_RefModel,), {"__module__": REF_MODEL}))
+    ref_model.get_model = lambda config: getattr(ref_model, config["name"])(**config)
+    ref_model.is_model_2d = lambda model: isinstance(model, ref_model.UNet2D)
+    had = sys.modules.get(REF_MODEL)
+    sys.modules[REF_MODEL] = ref_model
     yield ref_model
     import pytorch3dunet_b200 as P
     P.uninstall()
-    if added:
-        sys.path.remove(REF)
+    if had is None:
+        sys.modules.pop(REF_MODEL, None)
+    else:
+        sys.modules[REF_MODEL] = had
 
 
 def test_install_rebinds_get_model_and_keeps_2d_and_unsupported_on_the_reference(reference_pkg):
@@ -71,8 +66,7 @@ def test_install_rebinds_get_model_and_keeps_2d_and_unsupported_on_the_reference
             cfg.update(extra)
             mf = ref_model.get_model(cfg)
             assert type(mf) is ref_unet3d, extra
-            y = mf.eval()(torch.rand(1, 1, 8, 8, 8))   # and it runs (on the CPU, as the reference does)
-            assert y.shape == (1, 1, 8, 8, 8)
+            assert mf.kwargs == cfg, extra   # with the whole config, as the reference's get_model passes it
         assert P.install() is True  # idempotent
         assert P.uninstall() is True
         assert ref_model.get_model is ref_get_model and ref_model.UNet3D is ref_unet3d and caller.get_model is ref_get_model
@@ -83,20 +77,25 @@ def test_install_rebinds_get_model_and_keeps_2d_and_unsupported_on_the_reference
             sys.modules["pytorch3dunet.predict"] = had
 
 
-def test_engine_state_dict_loads_into_the_reference_and_back(reference_pkg):
-    """checkpoint compatibility both ways (utils.py:59-60 load_state_dict)"""
+def test_engine_state_dict_loads_into_the_reference_and_back():
+    """checkpoint compatibility both ways (utils.py:59-60 load_state_dict), against the state_dict the reference's get_model
+    builds for this config under torch.manual_seed(3)"""
     import pytorch3dunet_b200 as P
-    ref_model = reference_pkg
     cfg = dict(name="ResidualUNetSE3D", in_channels=1, out_channels=2, f_maps=16, num_levels=2, final_sigmoid=False)
-    torch.manual_seed(3)
-    ref = ref_model.get_model(cfg)
+    z = np.load(os.path.join(GOLDEN, "state_dict_resunetse3d_f16_l2_c2_seed3.npz"))
+    ref = {k[3:]: torch.from_numpy(z[k]) for k in z.files}
     torch.manual_seed(3)
     eng = P.get_model(cfg)
-    assert list(ref.state_dict().keys()) == list(eng.state_dict().keys())
-    for k, v in ref.state_dict().items():
+    # engine -> reference: the same names in the same order with the same shapes is what the reference's strict load checks
+    assert list(ref.keys()) == list(eng.state_dict().keys())
+    for k, v in ref.items():
         assert torch.equal(v, eng.state_dict()[k]), k     # same default init under the same seed
-    eng.load_state_dict(ref.state_dict())
-    ref.load_state_dict(eng.state_dict())
+    # reference -> engine
+    torch.manual_seed(4)
+    other = P.get_model(cfg)
+    other.load_state_dict(ref)
+    for k, v in other.state_dict().items():
+        assert torch.equal(v, ref[k]), k
 
 
 def test_unsupported_configurations_fail_at_construction_not_on_the_first_batch():
