@@ -215,6 +215,22 @@ int b200_pointwise_partials_count(int N, long long voxels, int Cout);
 int b200_pointwise_fwd(const void* x, int x_is_f32, const float* W, int transposed, const float* bias, int N, long long voxels,
                        int Cin, int Cout, void* y, float* partials, b200_stream_t s);
 /* partial rows [N*P][Cout*Cin + Cout] of dW, db; reduce with b200_reduce_rows */
+/* ---- gradient w.r.t. the fp32 network input (autograd of the first conv on x: buildingblocks.py:56, ResNetBlock.conv1 :251) ------------
+ * b200_input_dgrad_conv3: dx[n][ci][v] (fp32 NCDHW) = scale * sum_tap sum_co W[co][ci][tap] * dz[n, v - (tap-1), co]
+ *   dz: 16-bit NDHWC gradient of the conv output; W: fp32 (Cout,Cin,3,3,3), rounded to 16 bits like every other data-gradient operand.
+ *   Cin == 1 and Cout in {8,16,32}: warp-level MMA kernel; any other Cin (Cout % 8 == 0): CUDA-core kernel.  Fixed summation order, no
+ *   atomics.  partials (optional, then x = the NCDHW fp32 input is required): [N][P][Cin][2] = per-block (sum dx, sum dx*x),
+ *   P = b200_input_dgrad_partials_count, for the GroupNorm backward of a first layer that starts with a GroupNorm.
+ * b200_gn_bwd_apply_ncdhw_f32: out = scale * (A*dxhat + B*x + Cc), coef[N][C][3] = (A, B, Cc) from b200_gn_bwd_coeffs; out may alias dxhat.
+ * b200_pointwise_dgrad_f32: dx[n][ci][v] (fp32 NCDHW) = scale * sum_co W[co][ci] * dy[n,v,co]  (W fp32 (Cout,Cin)). */
+int b200_input_dgrad_partials_count(int N, int D, int H, int W, int Cin, int Cout);
+int b200_input_dgrad_conv3(const void* dz, const float* W, int N, int D, int H, int Wd, int Cin, int Cout, float scale, const float* x,
+                           float* dx, float* partials, b200_stream_t s);
+int b200_gn_bwd_apply_ncdhw_f32(const float* dxhat, const float* x, const float* coef, int N, int C, long long voxels, float scale,
+                                float* out, b200_stream_t s);
+int b200_pointwise_dgrad_f32(const void* dy, const float* W, int N, long long voxels, int Cin, int Cout, float scale, float* dx,
+                             b200_stream_t s);
+
 /* ---- "virtual concat" decoder convolution: conv3(GN(cat(enc, nearest_up2x(b)))) without the upsampled / concatenated tensor
  * (replaces F.interpolate + torch.cat + SingleConv of Decoder.forward, buildingblocks.py:466-497, when the encoder feature is
  * exactly 2x the low-res one).  y = conv3_enc(enc) [+bias, +R, act, stats: b200_conv3_fwd with pmode | B200_PMODE_PHASE_BIAS,

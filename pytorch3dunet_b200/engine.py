@@ -52,7 +52,7 @@ def _side_stream(device):
     return st
 PMODE_PHASE_BIAS = 0x100  # B200_PMODE_PHASE_BIAS (include/b200unet.h)
 HOST_PROF = None  # dict name -> [calls, seconds] when host profiling is on
-TIMED = {"b200_conv3_fwd", "b200_conv3_wgrad", "b200_conv3_up_phase_fwd", "b200_conv3_up_dgrad", "b200_conv3_up_dgrad_zs", "b200_conv3_up_wgrad",
+TIMED = {"b200_conv3_fwd", "b200_conv3_wgrad", "b200_input_dgrad_conv3", "b200_conv3_up_phase_fwd", "b200_conv3_up_dgrad", "b200_conv3_up_dgrad_zs", "b200_conv3_up_wgrad",
 
          "b200_pointwise_tc_fwd", "b200_pointwise_tc_wgrad", "b200_deconv_phase_fwd", "b200_deconv_phase_dgrad", "b200_deconv_phase_wgrad"}
 
@@ -111,13 +111,13 @@ class InputF32:
 
     __slots__ = ("t", "sums_src", "sums", "partials", "P", "requires_grad", "grad", "act", "slope", "grad_partials")
 
-    def __init__(self, t_ndhwc, ncdhw_src):
+    def __init__(self, t_ndhwc, ncdhw_src, requires_grad=False):
         self.t = t_ndhwc
         self.sums_src = ncdhw_src
         self.sums = None
         self.partials, self.P = None, 0
-        self.requires_grad = False
-        self.grad = None
+        self.requires_grad = requires_grad
+        self.grad = None        # fp32 NCDHW (the layout of the network input), unscaled: written by the first layer's backward
         self.grad_partials = None
         self.act, self.slope = ACT_NONE, 0.0
 
@@ -164,7 +164,7 @@ class VirtualCat:
 class Engine:
     """One forward (+ optional backward) pass.  Not reusable across passes."""
 
-    def __init__(self, device, impl=None, record=True, sink=None, operand_dtype="bf16", loss_scale=1.0):
+    def __init__(self, device, impl=None, record=True, sink=None, operand_dtype="bf16", loss_scale=1.0, data_only=False):
         # operand_dtype: the 16-bit type of activations and tensor-core operands ("bf16" | "fp16": two builds of the same kernels).
         # loss_scale (fp16): the seed gradient is multiplied by it and every parameter gradient divided by it, so that the backward
         # pass's activation gradients (~1e-7 for a mean-reduced loss over millions of voxels) stay inside fp16's range
@@ -172,6 +172,9 @@ class Engine:
         self.adt = torch.float16 if operand_dtype in ("fp16", "f16", "float16") else torch.bfloat16
         self.loss_scale = float(loss_scale)
         self.sink = sink      # optim.FlatParameters: parameter gradients are written straight into its flat buffer
+        # data_only: the backward computes input gradients only (every parameter frozen): no weight-gradient kernel, no parameter
+        # gradient, the GroupNorm-backward sums taken from the data gradients instead of from weight-gradient by-products
+        self.data_only = data_only
         self.sunk = set()
         self.device = device
         self.impl = default_impl() if impl is None else impl
@@ -260,6 +263,8 @@ class Engine:
         return torch.empty_like(like)
 
     def _add_param_grad(self, name, g):
+        if self.data_only:
+            return
         if self.loss_scale != 1.0:
             g.mul_(1.0 / self.loss_scale)   # (in place: also when g IS the flat-buffer view the kernel wrote into)
         if self.sink is not None:
@@ -359,7 +364,7 @@ class Engine:
         x.grad_partials = (parts, P, dxhat)
 
     # ---------------------------------------------------------------- input / output layout
-    def input_f32(self, x_ncdhw):
+    def input_f32(self, x_ncdhw, requires_grad=False):
         n, c, d, h, w = x_ncdhw.shape
         x_ncdhw = x_ncdhw.contiguous()
         if c == 1:
@@ -367,7 +372,51 @@ class Engine:
         else:
             t = self.empty((n, d, h, w, c), torch.float32)
             self.call("b200_ncdhw_f32_to_ndhwc_f32", _p(x_ncdhw), _p(t), n, c, d, h, w)
-        return InputF32(t, x_ncdhw)
+        return InputF32(t, x_ncdhw, requires_grad)
+
+    def set_input_grad(self, x, g):
+        """x.grad = g for the fp32 network input (fp32 NCDHW, unscaled).  Every model reads x in exactly one layer."""
+        if x.grad is not None:
+            raise B200Error("the fp32 network input is read by more than one layer: its gradient would need accumulating")
+        x.grad = g
+
+    def gn_bwd_coef_from_dgrad(self, dxhat, x, gamma, mean_rstd, groups, vox):
+        """GroupNorm-backward coefficients (A, B, C) of x from the data gradient dxhat itself (one pass over dxhat and x): what the
+        full backward takes from the weight-gradient by-products (b200_gn_bwd_sums_from_wgrad) when no weight gradient is computed"""
+        n, c = x.dims[0], x.dims[4]
+        P = self.L.query("b200_stats_partials_count", n, c, vox)
+        parts = self.empty((n, P, c, 2), torch.float32)
+        self.call("b200_stats2_ndhwc_bf16", _p(dxhat), _p(x.t), n, c, vox, _p(parts))
+        sums2 = self.empty((n, c, 2), torch.float64)
+        self.call("b200_partials_finalize", _p(parts), n, P, c, _p(sums2))
+        return self._gn_bwd_coef(sums2, gamma, mean_rstd, groups, vox, n, c)
+
+    def _gn_bwd_coef(self, sums2, gamma, mean_rstd, groups, vox, n, c):
+        coef = self.empty((n, c, 3), torch.float32)
+        dgamma, dbeta = self.empty((c,), torch.float32), self.empty((c,), torch.float32)   # (not published: parameters are frozen)
+        self.call("b200_gn_bwd_coeffs", _p(sums2), _p(gamma), _p(mean_rstd), groups, float(vox), n, c, _p(coef), _p(dgamma), _p(dbeta))
+        return coef
+
+    def input_dgrad_conv3(self, x, dz, W, coef, gn, mean_rstd, vox):
+        """gradient w.r.t. the fp32 network input x of the first 3x3x3 conv (csrc/input_grad.cu), GroupNorm backward included when the
+        layer starts with one; coef: the layer's GroupNorm-backward coefficients when the full backward already has them, else None"""
+        n, d, h, w, cin = x.dims
+        cout = W.shape[0]
+        inv = 1.0 / self.loss_scale
+        dx = self.empty((n, cin, d, h, w), torch.float32)
+        parts = None
+        if gn is not None and coef is None:
+            P = self.L.query("b200_input_dgrad_partials_count", n, d, h, w, cin, cout)
+            parts = self.empty((n, P, cin, 2), torch.float32)
+        self.call("b200_input_dgrad_conv3", _p(dz), _p(W), n, d, h, w, cin, cout, 1.0 if gn is not None else inv, _p(x.sums_src),
+                  _p(dx), _p(parts), flops=2.0 * n * vox * 27 * cin * cout, tag="dgrad_input")
+        if gn is not None:
+            if coef is None:
+                sums2 = self.empty((n, cin, 2), torch.float64)
+                self.call("b200_partials_finalize", _p(parts), n, parts.shape[1], cin, _p(sums2))
+                coef = self._gn_bwd_coef(sums2, gn[0].contiguous(), mean_rstd, gn[2], vox, n, cin)
+            self.call("b200_gn_bwd_apply_ncdhw_f32", _p(dx), _p(x.sums_src), _p(coef), n, cin, vox, inv, _p(dx))
+        self.set_input_grad(x, dx)
 
     def input_bf16(self, x_ncdhw, requires_grad):
         n, c, d, h, w = x_ncdhw.shape
@@ -446,13 +495,13 @@ class Engine:
                 dz = out.grad
                 if dz is None:
                     return
-                need_T = gn is not None or bias is not None
+                need_T = (gn is not None or bias is not None) and not self.data_only
                 T = wd = wd_ready = None
                 want_dx = x.requires_grad and not is_f32
                 if need_T or want_dx:
                     # second stream, under the weight-gradient kernel: the tap-flipped 16-bit weights of the data-gradient conv (needs
                     # only W) and the border tap sums T (only the reduction tail reads them)
-                    on_side = self.side_begin()
+                    on_side = self.side_begin() if not self.data_only else False
                     if want_dx:
                         wd = self.empty((27, cin, cout), self.adt)
                         self.call("b200_prep_dgrad_weights", _p(W), cin, cout, _p(wd))
@@ -460,56 +509,62 @@ class Engine:
                     if need_T:
                         T = self.border_tap_sums(out, dz, n, d, h, w, cout)
                     self.side_end(on_side)
-                wimpl = L.query("b200_conv3_wgrad_resolve_impl", self.impl, n, d, h, w, cin, cout, int(is_f32))
-                if wimpl < 0:
-                    raise B200Error("tcgen05 wgrad requested but unsupported for this shape")
-                S = L.query("b200_conv3_wgrad_splits", wimpl, n, d, h, w, cin, cout, int(is_f32))
-                G = self.empty((n, S, 27, cin, cout), torch.float32)
-                self.call("b200_conv3_wgrad", wimpl, _p(x.t), int(is_f32), _p(dz), n, d, h, w, cin, cout, _p(G),
-                          launches=1 if (wimpl == IMPL_TCGEN05 or S > 1) else 2, flops=2.0 * n * vox * 27 * cin * cout,
-                          tag=("wgrad_tc" if wimpl == IMPL_TCGEN05 else "wgrad_direct"), layer=name)
-                dW = torch.empty_like(W) if grad_sink is not None else self.grad_like(name + "conv.weight", W)
-                Gsum = self.empty((n, 1, 27, cin, cout), torch.float32) if gn is not None else None
-                db = torch.empty_like(bias) if bias is not None else None
-                coef = None
-                if gn is not None:
-                    sums2 = self.empty((n, cin, 2), torch.float64)
-                    coef = self.empty((n, cin, 3), torch.float32)
-                    dgamma, dbeta = torch.empty_like(gamma), torch.empty_like(beta)
-                on_side = self.side_begin()
-                self.call("b200_wgrad_finalize", _p(G), n, S, cin, cout, _p(ab), _p(T) if ab is not None else None, _p(dW), _p(Gsum))
-                if bias is not None:
-                    self.call("b200_bias_grad_from_T", _p(T), n, cout, _p(db))
-                if gn is not None:
-                    self.call("b200_gn_bwd_sums_from_wgrad", _p(Gsum), 1, _p(T), _p(W), n, cin, cout, _p(sums2))
-                    self.call("b200_gn_bwd_coeffs", _p(sums2), _p(gamma), _p(mean_rstd), groups, float(vox), n, cin,
-                              _p(coef), _p(dgamma), _p(dbeta))
-                tail = self.side_end(on_side)
-
-                def publish():  # main stream, after the join: hand the finished parameter gradients over
-                    if grad_sink is not None:
-                        grad_sink(dW)  # the weight is a derived tensor (e.g. the conv form of a ConvTranspose3d weight)
-                    else:
-                        self._add_param_grad(name + "conv.weight", dW)
-                    if bias is not None:
-                        self._add_param_grad(name + "conv.bias", db)
+                coef = tail = None
+                published = True
+                if not self.data_only:
+                    wimpl = L.query("b200_conv3_wgrad_resolve_impl", self.impl, n, d, h, w, cin, cout, int(is_f32))
+                    if wimpl < 0:
+                        raise B200Error("tcgen05 wgrad requested but unsupported for this shape")
+                    S = L.query("b200_conv3_wgrad_splits", wimpl, n, d, h, w, cin, cout, int(is_f32))
+                    G = self.empty((n, S, 27, cin, cout), torch.float32)
+                    self.call("b200_conv3_wgrad", wimpl, _p(x.t), int(is_f32), _p(dz), n, d, h, w, cin, cout, _p(G),
+                              launches=1 if (wimpl == IMPL_TCGEN05 or S > 1) else 2, flops=2.0 * n * vox * 27 * cin * cout,
+                              tag=("wgrad_tc" if wimpl == IMPL_TCGEN05 else "wgrad_direct"), layer=name)
+                    dW = torch.empty_like(W) if grad_sink is not None else self.grad_like(name + "conv.weight", W)
+                    Gsum = self.empty((n, 1, 27, cin, cout), torch.float32) if gn is not None else None
+                    db = torch.empty_like(bias) if bias is not None else None
+                    coef = None
                     if gn is not None:
-                        self._add_param_grad(gn[3], dgamma)
-                        self._add_param_grad(gn[4], dbeta)
-                published = not x.requires_grad or DEBUG is not None
-                if published:
-                    self.side_join(tail)
-                    publish()
-                if DEBUG is not None:
-                    DEBUG[name] = dict(dz=dz.clone(), T=None if T is None else T.clone(), G=G.clone(), dW=dW.clone(),
-                                       ab=None if ab is None else ab.clone(), x=x.t.clone(), y=out.t.clone(),
-                                       sums2=None if gn is None else sums2.clone(), coef=None if coef is None else coef.clone(),
-                                       mean_rstd=None if mean_rstd is None else mean_rstd.clone())
+                        sums2 = self.empty((n, cin, 2), torch.float64)
+                        coef = self.empty((n, cin, 3), torch.float32)
+                        dgamma, dbeta = torch.empty_like(gamma), torch.empty_like(beta)
+                    on_side = self.side_begin()
+                    self.call("b200_wgrad_finalize", _p(G), n, S, cin, cout, _p(ab), _p(T) if ab is not None else None, _p(dW), _p(Gsum))
+                    if bias is not None:
+                        self.call("b200_bias_grad_from_T", _p(T), n, cout, _p(db))
+                    if gn is not None:
+                        self.call("b200_gn_bwd_sums_from_wgrad", _p(Gsum), 1, _p(T), _p(W), n, cin, cout, _p(sums2))
+                        self.call("b200_gn_bwd_coeffs", _p(sums2), _p(gamma), _p(mean_rstd), groups, float(vox), n, cin,
+                                  _p(coef), _p(dgamma), _p(dbeta))
+                    tail = self.side_end(on_side)
+
+                    def publish():  # main stream, after the join: hand the finished parameter gradients over
+                        if grad_sink is not None:
+                            grad_sink(dW)  # the weight is a derived tensor (e.g. the conv form of a ConvTranspose3d weight)
+                        else:
+                            self._add_param_grad(name + "conv.weight", dW)
+                        if bias is not None:
+                            self._add_param_grad(name + "conv.bias", db)
+                        if gn is not None:
+                            self._add_param_grad(gn[3], dgamma)
+                            self._add_param_grad(gn[4], dbeta)
+                    published = not x.requires_grad or DEBUG is not None
+                    if published:
+                        self.side_join(tail)
+                        publish()
+                    if DEBUG is not None:
+                        DEBUG[name] = dict(dz=dz.clone(), T=None if T is None else T.clone(), G=G.clone(), dW=dW.clone(),
+                                           ab=None if ab is None else ab.clone(), x=x.t.clone(), y=out.t.clone(),
+                                           sums2=None if gn is None else sums2.clone(), coef=None if coef is None else coef.clone(),
+                                           mean_rstd=None if mean_rstd is None else mean_rstd.clone())
                 if residual is not None and residual.requires_grad:
                     self.act_bwd_into(residual, dz, cout, 0, self.empty(residual.t.shape, self.adt))
-                if x.requires_grad:
-                    if is_f32:
-                        raise NotImplementedError("gradient w.r.t. the fp32 network input is not provided by the engine")
+                if x.requires_grad and is_f32:
+                    if not published:
+                        self.side_join(tail)
+                        publish()
+                    self.input_dgrad_conv3(x, dz, W, coef, gn, mean_rstd, vox)
+                elif x.requires_grad:
                     self.side_join_event(wd_ready)
                     dimpl = L.query("b200_conv3_resolve_impl", self.impl, n, d, h, w, cout, cin, 0)
                     if dimpl < 0:
@@ -521,6 +576,8 @@ class Engine:
                     if not published:
                         self.side_join(tail)
                         publish()
+                    if gn is not None and coef is None:   # data-only backward
+                        coef = self.gn_bwd_coef_from_dgrad(dxhat, x, gamma, mean_rstd, groups, vox)
                     if coef is not None:
                         self.gn_bwd_apply(dxhat, x, coef, n, cin, vox)
                     else:
@@ -529,7 +586,7 @@ class Engine:
                         else:
                             x.grad = dxhat
                     if DEBUG is not None:
-                        DEBUG[name]["dx"] = dxhat.clone()
+                        DEBUG.setdefault(name, {})["dx"] = dxhat.clone()
                 out.grad = None
             self.tape.append(backward)
         return out
@@ -735,6 +792,10 @@ class Engine:
                     return
                 T = wd_enc = wd_up = wd_ready = None
                 want_dx = enc.requires_grad or low.requires_grad
+                if self.data_only:
+                    self._conv3_vcat_data_backward(vc, dz, W, gn, mean_rstd, name)
+                    out.grad = None
+                    return
                 if gn is not None or bias is not None or want_dx:
                     on_side = self.side_begin()   # under the two weight-gradient kernels
                     if want_dx:
@@ -783,55 +844,112 @@ class Engine:
                         self._add_param_grad(gn[4], dbeta)
                 self.side_join_event(wd_ready)
                 if enc.requires_grad:
-                    dimpl = L.query("b200_conv3_resolve_impl", self.impl, n, D, H, Wd, cout, c0, 0)
-                    if dimpl < 0:
-                        raise B200Error("tcgen05 dgrad requested but unsupported for this shape")
-                    ge = self.empty(enc.t.shape, self.adt)
-                    self.call("b200_conv3_fwd", dimpl, _p(dz), 0, _p(wd_enc), 1, None, 0, None, ACT_NONE, 0.0,
-                              n, D, H, Wd, cout, c0, _p(ge), 0, None, None, flops=2.0 * n * vox * 27 * c0 * cout,
-                              tag=("dgrad_tc" if dimpl == IMPL_TCGEN05 else "dgrad_direct"), layer=name)
+                    ge = self._vcat_dgrad_enc(vc, dz, wd_enc, cout, name)
                     if coef is not None:
                         if not published:
                             self.side_join(tail)
                             publish()
                             published = True
-                        if DEFER_GN_BWD and DEBUG is None and enc.pool_pending and enc.deferred is None and enc._grad is None:
-                            enc.deferred = (ge, coef[:, :c0].contiguous(), self)   # applied by the max-pool backward of enc
-                        else:
-                            self.gn_bwd_apply(ge, enc, coef[:, :c0].contiguous(), n, c0, vox)
-                    else:
-                        if enc.act != ACT_NONE or enc.grad is not None:
-                            self.act_bwd_into(enc, ge, c0, 0, ge)
-                        else:
-                            enc.grad = ge
+                    self._vcat_apply_enc(vc, ge, coef)
                 if low.requires_grad:
-                    gl = self.empty(low.t.shape, self.adt)
-                    if self.impl != IMPL_DIRECT and L.query("b200_conv3_up_dgrad_zs_supported", n, d, h, w, cout, c1):
-                        parts = self.empty((4,) + tuple(low.t.shape), self.adt)   # one partial gradient per in-plane parity of dz
-                        self.call("b200_conv3_up_dgrad_zs", _p(dz), _p(wd_up), n, d, h, w, cout, c1, _p(parts), _p(gl), launches=2,
-                                  flops=2.0 * n * lvox * 64 * c1 * cout, tag="dgrad_tc", layer=name)
-                        del parts
-                    else:
-                        self.call("b200_conv3_up_dgrad", _p(dz), _p(wd_up), n, d, h, w, cout, c1, _p(gl),
-                                  flops=2.0 * n * lvox * 64 * c1 * cout, tag="dgrad_tc", layer=name)
+                    gl = self._vcat_dgrad_low(vc, dz, wd_up, cout, name)
                     if coef is not None:
                         if not published:
                             self.side_join(tail)
                             publish()
                             published = True
-                        # d b[u] = sum over its 8 copies of (A dxhat + B x + C) = A sum(dxhat) + 8B b + 8C
-                        self.gn_bwd_apply(gl, low, (coef[:, c0:] * self._k188).contiguous(), n, c1, lvox)
-                    else:
-                        if low.act != ACT_NONE or low.grad is not None:
-                            self.act_bwd_into(low, gl, c1, 0, gl)
-                        else:
-                            low.grad = gl
+                    self._vcat_apply_low(vc, gl, coef)
                 if not published:
                     self.side_join(tail)
                     publish()
                 out.grad = None
             self.tape.append(backward)
         return out
+
+    def _vcat_dgrad_enc(self, vc, dz, wd_enc, cout, name):
+        """data gradient of conv3_enc: the raw (pre-GroupNorm-backward) gradient of the encoder part of the virtual concat"""
+        n, D, H, Wd, c0 = vc.enc.dims
+        dimpl = self.L.query("b200_conv3_resolve_impl", self.impl, n, D, H, Wd, cout, c0, 0)
+        if dimpl < 0:
+            raise B200Error("tcgen05 dgrad requested but unsupported for this shape")
+        ge = self.empty(vc.enc.t.shape, self.adt)
+        self.call("b200_conv3_fwd", dimpl, _p(dz), 0, _p(wd_enc), 1, None, 0, None, ACT_NONE, 0.0,
+                  n, D, H, Wd, cout, c0, _p(ge), 0, None, None, flops=2.0 * n * D * H * Wd * 27 * c0 * cout,
+                  tag=("dgrad_tc" if dimpl == IMPL_TCGEN05 else "dgrad_direct"), layer=name)
+        return ge
+
+    def _vcat_dgrad_low(self, vc, dz, wd_up, cout, name):
+        """data gradient of conv3_up: the gradient of the low-res tensor summed over its 8 copies in the virtual upsample"""
+        n, d, h, w, c1 = vc.low.dims
+        lvox = d * h * w
+        L = self.L
+        gl = self.empty(vc.low.t.shape, self.adt)
+        if self.impl != IMPL_DIRECT and L.query("b200_conv3_up_dgrad_zs_supported", n, d, h, w, cout, c1):
+            parts = self.empty((4,) + tuple(vc.low.t.shape), self.adt)   # one partial gradient per in-plane parity of dz
+            self.call("b200_conv3_up_dgrad_zs", _p(dz), _p(wd_up), n, d, h, w, cout, c1, _p(parts), _p(gl), launches=2,
+                      flops=2.0 * n * lvox * 64 * c1 * cout, tag="dgrad_tc", layer=name)
+            del parts
+        else:
+            self.call("b200_conv3_up_dgrad", _p(dz), _p(wd_up), n, d, h, w, cout, c1, _p(gl),
+                      flops=2.0 * n * lvox * 64 * c1 * cout, tag="dgrad_tc", layer=name)
+        return gl
+
+    def _vcat_apply_enc(self, vc, ge, coef):
+        enc = vc.enc
+        n, D, H, Wd, c0 = enc.dims
+        if coef is not None:
+            if DEFER_GN_BWD and DEBUG is None and enc.pool_pending and enc.deferred is None and enc._grad is None:
+                enc.deferred = (ge, coef[:, :c0].contiguous(), self)   # applied by the max-pool backward of enc
+            else:
+                self.gn_bwd_apply(ge, enc, coef[:, :c0].contiguous(), n, c0, D * H * Wd)
+        else:
+            if enc.act != ACT_NONE or enc.grad is not None:
+                self.act_bwd_into(enc, ge, c0, 0, ge)
+            else:
+                enc.grad = ge
+
+    def _vcat_apply_low(self, vc, gl, coef):
+        low = vc.low
+        n, d, h, w, c1 = low.dims
+        c0 = vc.enc.dims[4]
+        if coef is not None:
+            # d b[u] = sum over its 8 copies of (A dxhat + B x + C) = A sum(dxhat) + 8B b + 8C
+            self.gn_bwd_apply(gl, low, (coef[:, c0:] * self._k188).contiguous(), n, c1, d * h * w)
+        else:
+            if low.act != ACT_NONE or low.grad is not None:
+                self.act_bwd_into(low, gl, c1, 0, gl)
+            else:
+                low.grad = gl
+
+    def _conv3_vcat_data_backward(self, vc, dz, W, gn, mean_rstd, name):
+        """input-gradient-only backward of the virtual-concat convolution.  With a GroupNorm in front, its backward sums over the
+        concatenated tensor come from the two raw data gradients: sum over the full-res voxels of the upsampled part of (dxhat, dxhat*x)
+        equals sum over the low-res voxels of (gl, gl*b), since gl already sums each voxel's 8 copies"""
+        enc, low = vc.enc, vc.low
+        n, D, H, Wd, c0 = enc.dims
+        c1 = low.dims[4]
+        cout = W.shape[0]
+        wd_enc = self.empty((27, c0, cout), self.adt)
+        wd_up = self.empty((64, c1, cout), self.adt)
+        self.call("b200_upcat_prep_dgrad_weights", _p(W), c0, c1, cout, _p(wd_enc), _p(wd_up))
+        ge = self._vcat_dgrad_enc(vc, dz, wd_enc, cout, name) if (enc.requires_grad or gn is not None) else None
+        gl = self._vcat_dgrad_low(vc, dz, wd_up, cout, name) if (low.requires_grad or gn is not None) else None
+        coef = None
+        if gn is not None:
+            sums = []
+            for g, t in ((ge, enc), (gl, low)):
+                tn, td, th, tw, tc = t.dims
+                P = self.L.query("b200_stats_partials_count", tn, tc, td * th * tw)
+                parts = self.empty((tn, P, tc, 2), torch.float32)
+                self.call("b200_stats2_ndhwc_bf16", _p(g), _p(t.t), tn, tc, td * th * tw, _p(parts))
+                s2 = self.empty((tn, tc, 2), torch.float64)
+                self.call("b200_partials_finalize", _p(parts), tn, P, tc, _p(s2))
+                sums.append(s2)
+            coef = self._gn_bwd_coef(torch.cat(sums, dim=1).contiguous(), gn[0].contiguous(), mean_rstd, gn[2], D * H * Wd, n, c0 + c1)
+        if enc.requires_grad:
+            self._vcat_apply_enc(vc, ge, coef)
+        if low.requires_grad:
+            self._vcat_apply_low(vc, gl, coef)
 
     def _upcat_materialize(self, enc, x, want_stats=True, mode="nearest"):
         n, D, H, W, c0 = enc.dims
@@ -888,7 +1006,9 @@ class Engine:
                 dy = out.grad
                 if dy is None:
                     return
-                if tc:
+                if self.data_only:
+                    pass   # frozen parameters: no weight or bias gradient
+                elif tc:
                     S = self.L.query("b200_pointwise_tc_wgrad_splits", n, vox, cin, cout)
                     G = self.empty((n * S, cin * cout), torch.float32)
                     self.call("b200_pointwise_tc_wgrad", _p(x.t), _p(dy), n, vox, cin, cout, _p(G),
@@ -908,9 +1028,11 @@ class Engine:
                     self._add_param_grad(wname, red[: cout * cin].reshape(W.shape))
                     if bias is not None:
                         self._add_param_grad(bname, red[cout * cin:].clone())
-                if x.requires_grad:
-                    if is_f32:
-                        raise NotImplementedError("gradient w.r.t. the fp32 network input is not provided by the engine")
+                if x.requires_grad and is_f32:
+                    dx = self.empty((n, cin, d, h, w), torch.float32)
+                    self.call("b200_pointwise_dgrad_f32", _p(dy), _p(W2), n, vox, cin, cout, 1.0 / self.loss_scale, _p(dx))
+                    self.set_input_grad(x, dx)
+                elif x.requires_grad:
                     g = self.empty(x.t.shape, self.adt)
                     if tc:
                         wqt = self.empty((cin, cout), self.adt)
@@ -1016,13 +1138,14 @@ class Engine:
                     return
                 gp = self.empty((n, D, H, W_, cout), self.adt)
                 self.call("b200_shift_fold_bwd", _p(g), n, D, H, W_, cout, _p(gp))
-                S = self.L.query("b200_deconv_phase_wgrad_splits", n, d, h, w, cout, cin)
-                Q = self.empty((n * S, 27, cout, cin), torch.float32)
-                self.call("b200_deconv_phase_wgrad", _p(gp), _p(x.t), n, d, h, w, cout, cin, _p(Q),
-                          flops=2.0 * n * d * h * w * 27 * cin * cout, tag="wgrad_tc", layer=wname)
-                dWt = self.grad_like(wname, Wt)
-                self.call("b200_deconv_phase_wgrad_finalize", _p(Q), n * S, cin, cout, _p(dWt))
-                self._add_param_grad(wname, dWt)
+                if not self.data_only:
+                    S = self.L.query("b200_deconv_phase_wgrad_splits", n, d, h, w, cout, cin)
+                    Q = self.empty((n * S, 27, cout, cin), torch.float32)
+                    self.call("b200_deconv_phase_wgrad", _p(gp), _p(x.t), n, d, h, w, cout, cin, _p(Q),
+                              flops=2.0 * n * d * h * w * 27 * cin * cout, tag="wgrad_tc", layer=wname)
+                    dWt = self.grad_like(wname, Wt)
+                    self.call("b200_deconv_phase_wgrad_finalize", _p(Q), n * S, cin, cout, _p(dWt))
+                    self._add_param_grad(wname, dWt)
                 if x.requires_grad:
                     gx = self.empty(x.t.shape, self.adt)
                     self.call("b200_deconv_phase_dgrad", _p(gp), _p(wd), n, d, h, w, cout, cin, _p(gx),
@@ -1073,7 +1196,8 @@ class Engine:
                 sums2 = self.empty((n, c, 2), torch.float64)
                 self.call("b200_partials_finalize", _p(part), n, P, c, _p(sums2))
                 dbs = self.empty((1,), torch.float32)
-                self.call("b200_reduce_rows", _p(dbs_part), n * P, 1, _p(dbs))
+                if not self.data_only:
+                    self.call("b200_reduce_rows", _p(dbs_part), n * P, 1, _p(dbs))
                 coef = self.empty((n, c, 3), torch.float32)
                 dW1, db1 = torch.empty_like(W1), torch.empty_like(b1)
                 dW2, db2 = torch.empty_like(W2), torch.empty_like(b2)
@@ -1112,11 +1236,12 @@ class Engine:
             partials = self.empty((n * P, K), torch.float32)
             dz = self.empty(x.t.shape, self.adt)
             self.call("b200_final_conv_bwd", _p(dlogits), _p(x.t), n, vox, c, _p(W2), cout, x.act, x.slope, _p(dz), _p(partials))
-            red = self.empty((K,), torch.float32)
-            self.call("b200_reduce_rows", _p(partials), n * P, K, _p(red))
-            self._add_param_grad(wname, red[: cout * c].reshape(W.shape))
-            if bias is not None:
-                self._add_param_grad(bname, red[cout * c:].clone())
+            if not self.data_only:   # (the per-block dW / db partials are a by-product of the dz kernel)
+                red = self.empty((K,), torch.float32)
+                self.call("b200_reduce_rows", _p(partials), n * P, K, _p(red))
+                self._add_param_grad(wname, red[: cout * c].reshape(W.shape))
+                if bias is not None:
+                    self._add_param_grad(bname, red[cout * c:].clone())
             self.accumulate_grad(x, dz)
         return logits, probs, backward
 

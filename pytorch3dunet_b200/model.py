@@ -71,8 +71,12 @@ class _EngineFn(torch.autograd.Function):
         # Function.forward: the caller's mode comes in as an argument.  Under torch.no_grad() (the predictor's path,
         # reference predictor.py:164) nothing is taped, so no closure pins a layer's activations.
         needs_grad = bool(grad_mode) and any(ctx.needs_input_grad[6:])
+        # every parameter frozen, an input requiring grad (a frozen network used as a loss, saliency maps, ...): the backward computes the
+        # input gradient only -- no weight-gradient kernel, no parameter gradient, the flat gradient buffer is not touched
+        data_only = needs_grad and not any(ctx.needs_input_grad[6 + n_inputs:])
         with torch.cuda.device(x0.device):
-            eng = E.Engine(x0.device, record=needs_grad, sink=sink, operand_dtype=opts[0], loss_scale=opts[1] if needs_grad else 1.0)
+            eng = E.Engine(x0.device, record=needs_grad, sink=None if data_only else sink, operand_dtype=opts[0],
+                           loss_scale=opts[1] if needs_grad else 1.0, data_only=data_only)
             sd = dict(zip(names, params))
             in_req = [needs_grad and bool(g) for g in ctx.needs_input_grad[6:6 + n_inputs]]
             outs, seed, input_grads = program(eng, [t.detach() for t in inputs], sd, in_req)
@@ -91,6 +95,10 @@ class _EngineFn(torch.autograd.Function):
         eng = ctx.eng
         if eng is None or not eng.record:
             raise RuntimeError("b200 engine: backward called twice or without a recorded forward")
+        if torch.is_grad_enabled():
+            # autograd runs backward with grad mode on exactly when create_graph=True: the engine's gradients are not themselves
+            # differentiable, so a second-order term would silently come out as zero
+            raise RuntimeError("b200 engine: double backward (create_graph=True) is not supported")
         with torch.cuda.device(ctx.device):
             eng.stream = torch.cuda.current_stream(ctx.device).cuda_stream
             l0 = eng.launches
@@ -549,9 +557,7 @@ class AbstractUNet(nn.Module):
             x = x.float()
 
         def program(eng, ins, sd, in_req):
-            if in_req[0]:
-                raise NotImplementedError("gradient w.r.t. the network input is not provided by the b200 engine")
-            xin = eng.input_f32(ins[0])
+            xin = eng.input_f32(ins[0], requires_grad=in_req[0])
             logits, probs, final_bwd = run_unet(eng, xin, sd, spec)
             final = spec["is_segmentation"]
             # the closure must not hold the tensor OBJECT that forward returns: that object gets grad_fn = this autograd node,
@@ -570,8 +576,14 @@ class AbstractUNet(nn.Module):
                     g_logits = t if g_logits is None else g_logits + t
                 if g_logits is not None:
                     final_bwd(g_logits * eng.loss_scale if eng.loss_scale != 1.0 else g_logits)
+
+            def input_grads(eng):
+                # fp32 NCDHW, unscaled; zeros when the loss did not depend on the output
+                if not in_req[0]:
+                    return [None]
+                return [xin.grad if xin.grad is not None else torch.zeros_like(ins[0])]
             outs = [logits, probs] if final else [logits]
-            return outs, seed, lambda eng: [None]
+            return outs, seed, input_grads
         res = _run(self, program, [x])
         logits = res[0]
         out = res[1] if spec["is_segmentation"] else logits
